@@ -2,6 +2,7 @@
 """bench.py -- B-reps/sec of the 1000-step-per-stage ABC cascade (BASELINE.json), one process per GPU.
 
     python bench.py --gpus 1 --steps 3 --warmup 3
+    python bench.py --gpus 1 --steps 3 --warmup 3 --dump-outputs DIR   # + the last timed step's outputs as DIR/*.npy
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
     python bench.py --impl reference ...        # the reference's own classes on the host cores (baseline/_ref), same metric
 
@@ -32,6 +33,7 @@ import torch  # noqa: E402
 METRIC = "B-reps/sec (1000-step ABC cascade)"
 UNIT = "B-reps/s"
 KINDS = ("surfpos", "surfz", "edgepos", "edgez")
+DUMP_BYTES = 64 * 10**6
 
 
 def parse():
@@ -58,7 +60,15 @@ def parse():
                          "1000-step DDPM, 30 face tokens, batch 64 (first stage only), eager loop vs CUDA-graph replay")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the cascade outputs of the last one as DIR/<name>.npy (float32; rank 0; "
+                         f"when they exceed {DUMP_BYTES // 10**6} MB together, the same seeded sample of batch rows of each)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.workload != "cascade"):
+        ap.error("--dump-outputs applies to the cascade workload of --impl b200")
+    return args
 
 
 def peaks():
@@ -179,6 +189,19 @@ def best_cpu_threads():
         if best_t is None or dt < best_t:
             best, best_t = k, dt
     return best
+
+
+def dump_outputs(out, d):
+    """every output of Cascade.run has the batch first: keep the same seeded rows of each so that the sample stays one
+    set of whole B-reps, as many as fit DUMP_BYTES (npy headers included)"""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    B = next(iter(out.values())).shape[0]
+    row_bytes = sum(v[0].numel() * 4 for v in out.values())
+    n = min(B, (DUMP_BYTES - 4096 * len(out)) // row_bytes)
+    rows = torch.randperm(B, generator=torch.Generator().manual_seed(0))[:n].sort().values
+    for k, v in out.items():
+        np.save(os.path.join(d, f"{k}.npy"), v[rows.to(v.device)].float().cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------------ clocks sampler
@@ -373,6 +396,8 @@ def main():
     ms = timed(step_resident, args.steps)
     launches = _ffi.lib().bg_launch_count() + _ffi.replayed_launches - l0      # host launches + kernels inside graph replays
     clk = clocks.finish()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last["out"], args.dump_outputs)
     scale = 1000.0 / T if args.schedule == "ddpm" else 1.0     # the shipped hybrid is run literally
     # the two VAE decodes run once per cascade whatever T is: time them alone and keep them out of the 1000/T scaling
     ms_dec = 0.0

@@ -226,14 +226,23 @@ def test_valid_token_flops_reduce_to_dense_when_nothing_is_masked():
 
 
 def test_reference_loader_runs_the_reference_classes_when_available():
+    """the reference's own SurfPosNet, imported by the loader, stored by tests/golden/make_golden_loader.py: the oracle
+    restatement reproduces it everywhere, and the loader does wherever the reference's network.py is present"""
+    import make_golden_loader as G
     from oracle.reference_loader import load_reference_network, reference_dir
-    if reference_dir() is None:
-        pytest.skip("neither /root/reference nor baseline/_ref present")
-    net = load_reference_network()
-    m = net.SurfPosNet(False).eval()
+    ref = np.load(os.path.join(ROOT, "tests", "golden", "loader_golden.npz"))["surfpos"]
+    assert ref.shape == (1, 4, 6)
+    sd, x, t = G.case()
     with torch.no_grad():
-        y = m(torch.zeros(1, 4, 6), torch.tensor([3]), None)
-    assert y.shape == (1, 4, 6)
+        y = O.surfpos_forward(sd, x, t).numpy()
+    assert np.abs(y - ref).max() < 1e-5 * np.abs(ref).max()
+    if reference_dir() is not None:
+        m = load_reference_network().SurfPosNet(False)
+        m.load_state_dict(sd)
+        m.eval()
+        with torch.no_grad():
+            y = m(x, t, None).numpy()
+        assert np.abs(y - ref).max() < 1e-5 * np.abs(ref).max()
 
 
 def test_load_cascade_and_config_from_eval_args():
